@@ -87,7 +87,7 @@ typedef struct lfm_edm_desc {
  * latent_channels 4, out_channels 3).  diffusers is a third-party dependency outside /root/reference: the architecture
  * is restated in oracle/vae.py (parity unpinned). */
 typedef struct lfm_vae_desc {
-    int32_t latent_size;            /* latent side = image_size // 8: 16, 32 (256 x 256 images; the LFM presets) */
+    int32_t latent_size;            /* latent side = image_size // 8: 16, 32 (256 x 256 images; the LFM presets), 64 (512 x 512) */
     int32_t latent_channels;        /* 4 */
     int32_t out_channels;           /* 3 */
     int32_t n_blocks;               /* number of entries used in block_out_channels */

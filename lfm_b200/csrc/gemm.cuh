@@ -31,13 +31,14 @@ struct GemmEpi {
     int rows_per_sample;  // tokens per sample (b = row / rows_per_sample)
     // Optional (pair kernel, EPI_BIAS_F32): GroupNorm statistics of the OUTPUT accumulated in the epilogue -
     // bins[((row / gn_hw) * kGnBinReplicas + r) * 64 + 2 g + {0,1}] += {sum, sum of squares} of group g = column / gn_cpg, as
-    // 2^28 fixed point (integer atomics => the result does not depend on the order of arrival: deterministic).  r is any of
+    // gn_scale fixed point (integer atomics => the result does not depend on the order of arrival: deterministic).  r is any of
     // kGnBinReplicas copies (chosen per warp; the consumer adds them up - integers, so still exact): persistent CTAs walk the
     // tiles of ONE image together, and with a single copy every atomic of the chip queued on the same four 128-byte lines
     // (a 128-channel 256 x 256 VAE layer: 2.1 M atomics, +525 us on a 410 us convolution; profiles/r2l_vae_launches.md).
     unsigned long long* gn_bins = nullptr;
     int gn_cpg = 0;
     int gn_hw = 1;
+    float gn_scale = 268435456.0f;  // fixed-point scale of this statistics slot (gn_fix_scale); the consumer reads GnApplyArgs::bins_unit
     // Pair kernel: walk the M blocks from the last to the first.  Consecutive kernels of a network alternate
     // direction so that each one starts on the rows its producer touched LAST - the part still resident in L2.
     int reverse_m = 0;
@@ -67,7 +68,16 @@ struct GemmEpi {
     int ln_stride = 0;
 };
 constexpr int kGnBinReplicas = 16;
-constexpr double kGnFixScale = 268435456.0;  // 2^28
+// Fixed-point scale of the fused GroupNorm statistics, chosen per slot from n = H * W * C / 32, the elements of one
+// (image, group).  The replicas are added as long long, so the sum of squares n * E[x^2] must stay below 2^63 / scale:
+// 2^28 (every layer with n <= 2^19 - all of the 256-pixel decode and the UNets) allows an rms of 2^17.5 / sqrt(n), 256 at
+// n = 2^19, 181 at 2^20.  The 512-pixel decode's last stage reaches n = 2^20 (2^21 with LFM_UNET_FUSE_OUT=1): 2^22 there,
+// rms up to 1448 / 1024.  One atomic rounds by at most 0.5 / scale (2^-23 at 2^22): negligible next to sums of 2^20 values.
+constexpr double kGnFixScale = 268435456.0;   // 2^28
+constexpr double kGnFixScaleWide = 4194304.0; // 2^22
+constexpr long long kGnFixWideN = 1 << 19;    // n above which a slot uses kGnFixScaleWide
+constexpr double kGnMinRms = 256.0;           // the host refuses a slot whose scale allows a smaller rms than this
+__host__ __device__ constexpr double gn_fix_scale(long long n) { return n <= kGnFixWideN ? kGnFixScale : kGnFixScaleWide; }
 
 constexpr int kGemmBlockM = 128;
 constexpr int kGemmBlockK = 64;  // 64 bf16 = one 128-byte swizzle row

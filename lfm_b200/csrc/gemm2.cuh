@@ -73,8 +73,8 @@ LFM_DEVICE void tma_load_4d_2sm(void* smem_dst, const CUtensorMap* m, uint64_t* 
 
 // Implicit-GEMM convolution geometry (taps == 0: plain GEMM, A is a 2-D [M, K] matrix).
 // Output pixels are flattened (b, h, w) row-major; a CTA's 128 output rows are whole image rows (W * rows == 128),
-// whole images (H * W divides 128) or one 128-pixel segment of an image row (W = 256: the VAE decoder's last stage),
-// so the matching input window of tap (r, s) is ONE 4-D box.
+// whole images (H * W divides 128) or one 128-pixel segment of an image row (W = 256 or 512, a multiple of 128: the last
+// stages of the VAE decoder - 2 or 4 segments per row), so the matching input window of tap (r, s) is ONE 4-D box.
 struct ConvGeom {
     int taps;     // 0 (GEMM), 9 (3x3, pad 1)
     int cblocks;  // C_in / 64
@@ -206,7 +206,7 @@ LFM_DEVICE float halving_reduce(float (&v)[V], int lane) {
     return v[0];  // the total of value (lane >> (5 - log2 V)); every lane of that group of lanes holds it
 }
 template <int CPG>
-LFM_DEVICE void gn_accumulate_chunk(const float* f, bool row_ok, int n0, unsigned long long* bins_b, int lane) {
+LFM_DEVICE void gn_accumulate_chunk(const float* f, bool row_ok, int n0, unsigned long long* bins_b, int lane, double scale) {
     constexpr int NG = CPG >= 32 ? 1 : 32 / CPG;   // groups inside this chunk
     constexpr int W = CPG >= 32 ? 32 : CPG;        // columns per group inside this chunk
     constexpr int V = 2 * NG;                      // {sum, sum of squares} per group
@@ -228,7 +228,7 @@ LFM_DEVICE void gn_accumulate_chunk(const float* f, bool row_ok, int n0, unsigne
     if ((lane & ((1 << SH) - 1)) == 0) {
         const int idx = lane >> SH;
         const int g = (n0 + (idx >> 1) * W) / CPG;
-        atomicAdd(bins_b + 2 * g + (idx & 1), static_cast<unsigned long long>(__double2ll_rn(static_cast<double>(total) * kGnFixScale)));
+        atomicAdd(bins_b + 2 * g + (idx & 1), static_cast<unsigned long long>(__double2ll_rn(static_cast<double>(total) * scale)));
     }
 }
 LFM_DEVICE void gn_accumulate(const float* f, const GemmEpi& ep, int row, int M, int n0, int N, int lane) {
@@ -237,12 +237,13 @@ LFM_DEVICE void gn_accumulate(const float* f, const GemmEpi& ep, int row, int M,
     unsigned long long* bins_b = ep.gn_bins + (static_cast<size_t>((row < M ? row : M - 1) / ep.gn_hw) * kGnBinReplicas + rep) * 64;
     bins_b = reinterpret_cast<unsigned long long*>(__shfl_sync(0xffffffffu, reinterpret_cast<unsigned long long>(bins_b), 0));
     const bool ok = row < M;
+    const double sc = static_cast<double>(ep.gn_scale);
     switch (ep.gn_cpg) {
-        case 4: gn_accumulate_chunk<4>(f, ok, n0, bins_b, lane); break;
-        case 8: gn_accumulate_chunk<8>(f, ok, n0, bins_b, lane); break;
-        case 16: gn_accumulate_chunk<16>(f, ok, n0, bins_b, lane); break;
-        case 32: gn_accumulate_chunk<32>(f, ok, n0, bins_b, lane); break;
-        case 64: gn_accumulate_chunk<64>(f, ok, n0, bins_b, lane); break;
+        case 4: gn_accumulate_chunk<4>(f, ok, n0, bins_b, lane, sc); break;
+        case 8: gn_accumulate_chunk<8>(f, ok, n0, bins_b, lane, sc); break;
+        case 16: gn_accumulate_chunk<16>(f, ok, n0, bins_b, lane, sc); break;
+        case 32: gn_accumulate_chunk<32>(f, ok, n0, bins_b, lane, sc); break;
+        case 64: gn_accumulate_chunk<64>(f, ok, n0, bins_b, lane, sc); break;
         default: break;
     }
 }
@@ -458,7 +459,7 @@ gemm2_bf16_tcgen05(const __grid_constant__ CUtensorMap tmap_a,   // A [M, K], bo
                 if (cg.taps != 0) {
                     img0 = row_a / cg.HW;
                     h0 = (row_a % cg.HW) / cg.W;
-                    w0 = row_a % cg.W;  // non-zero only when an image row is wider than the 128-pixel tile (W = 256)
+                    w0 = row_a % cg.W;  // non-zero only when an image row is wider than the 128-pixel tile (W = 256, 512)
                 }
                 const int ks = ksplit > 1 ? item % ksplit : 0;
                 const int kb0 = ks * kb_per, kb1 = min(num_kb, kb0 + kb_per);

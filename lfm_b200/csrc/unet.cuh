@@ -89,6 +89,7 @@ struct GnApplyArgs {
     const __nv_bfloat16* src_bf16;  // nullptr, or the source as bf16 [B, HW, C] (conv1's output when its fp32 statistics were
                                     // taken in that conv's epilogue: half the bytes to write and to read back)
     int HW, C, nchunk;
+    float bins_unit;                 // 1 / the fixed-point scale the producer of `bins` used (GemmEpi::gn_scale): 2^-28 or 2^-22
     const double* partial;
     const unsigned long long* bins;  // nullptr, or fixed-point {sum, sumsq} per (sample, group) from the producing conv
     const float* gamma;
@@ -114,8 +115,8 @@ LFM_DEVICE void gn_coefficients(const GnApplyArgs& a, int b, float* s_coef, floa
                 si += static_cast<long long>(bp[0]);
                 qi += static_cast<long long>(bp[1]);
             }
-            S = static_cast<double>(si) / 268435456.0;
-            Q = static_cast<double>(qi) / 268435456.0;
+            S = static_cast<double>(si) * static_cast<double>(a.bins_unit);  // a power of two: exact
+            Q = static_cast<double>(qi) * static_cast<double>(a.bins_unit);
         } else {
             for (int c = 0; c < a.nchunk; ++c) {  // fixed order => deterministic
                 S += a.partial[(static_cast<size_t>(b) * a.nchunk + c) * 64 + 2 * threadIdx.x];

@@ -1,8 +1,9 @@
 """Small end-to-end run for compute-sanitizer (memcheck / racecheck / synccheck): every native family once, at sizes the
 instrumented run finishes in minutes - mini DiT (forward with labels, CFG Heun from the step graph, dopri5 from the step
 graph, LayerNorm finisher path), mini ADM UNetModel, mini EDM DhariwalUNet (resampling blocks, both attention kernels),
-the VAE decoder at 128 x 128 (batched attention GEMMs, 128-pixel conv tiles) with the fused uint8 post-processing.
-  compute-sanitizer --tool memcheck  python scripts/sanitizer_run.py
+the VAE decoder at 128 x 128 (batched attention GEMMs, 128-pixel conv tiles) with the fused uint8 post-processing, and
+at 512 x 512 (vae512: two images; 4096-token attention, four row segments per image row, 2^22 fixed-point statistics).
+  compute-sanitizer --tool memcheck  python scripts/sanitizer_run.py [dit unet edm vae vae512]
   compute-sanitizer --tool racecheck python scripts/sanitizer_run.py"""
 import os
 import sys
@@ -16,7 +17,7 @@ import lfm_b200  # noqa: E402
 from lfm_b200.synthetic import synthetic_edm_state_dict, synthetic_state_dict, synthetic_unet_state_dict  # noqa: E402
 
 dev = torch.device("cuda:0")
-which = sys.argv[1:] or ["dit", "unet", "edm", "vae"]
+which = sys.argv[1:] or ["dit", "unet", "edm", "vae", "vae512"]
 x = torch.randn(3, 4, 32, 32, device=dev)
 res = {}
 if "dit" in which:
@@ -50,5 +51,11 @@ if "vae" in which:
     vae = vae.to(dev)
     u8 = vae.decode_to_uint8(torch.randn(2, 4, 16, 16, device=dev))
     res["vae"] = float(u8.float().mean())
+if "vae512" in which:
+    vae = lfm_b200.AutoencoderKL(max_batch=2)
+    vae.load_state_dict(lfm_b200.synthetic_vae_state_dict(vae, 2), strict=True)
+    vae = vae.to(dev)
+    u8 = vae.decode_to_uint8(torch.randn(2, 4, 64, 64, device=dev))
+    res["vae512"] = float(u8.float().mean())
 torch.cuda.synchronize()
 print("ok", res)
